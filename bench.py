@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the OmniVGGT hot path (BASELINE.json metric: view-sets/sec, N-view 518^2 batches).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config cfg1..cfg5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config cfg1..cfg5] [--dump-outputs DIR]
 
 One "step" = the full OmniVGGT.forward over this rank's share of the workload.  Workloads (BASELINE.json configs[0..4]):
   cfg1  1 scene x 4 views @ 518^2, images only
@@ -11,6 +11,8 @@ One "step" = the full OmniVGGT.forward over this rank's share of the workload.  
   cfg5  1 scene x 24 views @ 518^2, partial depth_gt_index / camera_gt_index
 cfg1/2/3/5 under torchrun: weak scaling, one independent view-set per rank per step; weights broadcast once from rank 0 (NCCL).
 Prints ONE JSON line on rank 0 (DESIGN.md section "Measurement" defines the fields).
+--dump-outputs DIR writes rank 0's predictions of the last timed step to DIR (see dump_outputs); inputs and weights are
+seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -21,6 +23,7 @@ import statistics
 import subprocess
 import sys
 import time
+import zlib
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
@@ -40,6 +43,7 @@ CONFIGS = {
                  desc="cfg5: 1 scene x 24 views @ 518x518, partial depth / camera aux, per GPU per step (BASELINE.json configs[4])"),
 }
 OUT_KEYS = ("pose_enc", "depth", "depth_conf", "world_points", "world_points_conf")
+DUMP_BYTES = 60_000_000          # payload cap of --dump-outputs (with the .npy headers the files stay under 64 MB)
 
 
 def measured_peaks():
@@ -67,6 +71,33 @@ def synth_inputs(B, S, seed):
     mask = (torch.rand(B, S, IMG, IMG, generator=g) > 0.2).float()
     depth = (0.5 + 4.0 * torch.rand(B, S, IMG, IMG, 1, generator=g)) * mask[..., None]
     return dict(images=images, extrinsics=extr, intrinsics=intr, depth=depth, mask=mask)
+
+
+def dump_outputs(outs, directory, limit=DUMP_BYTES):
+    """Write what one step returned to its caller as ``directory/<name>.npy`` (float32).  ``outs`` holds the output dict of
+    every forward call of the step; the calls are concatenated along the scene axis, ``pose_enc_list`` is written as
+    ``pose_enc_list.<i>``.  ``images`` (the caller's own input, handed back unchanged) and non-tensor entries are skipped.
+    If the arrays exceed ``limit`` bytes together, the smallest are kept whole and every array larger than its share of
+    what is left is replaced by a sample of its flattened elements: the sorted indices drawn without replacement by
+    ``numpy.random.default_rng(zlib.crc32(name))``, so that the same arguments give the same sample on every run."""
+    import numpy as np
+    import torch
+    arrays = {}
+    for k, v in outs[0].items():
+        if k == "pose_enc_list":
+            for i in range(len(v)):
+                arrays[f"{k}.{i}"] = torch.cat([o[k][i] for o in outs]).float().cpu().numpy()
+        elif torch.is_tensor(v) and k != "images":
+            arrays[k] = torch.cat([o[k] for o in outs]).float().cpu().numpy()
+    os.makedirs(directory, exist_ok=True)
+    left = limit
+    for n, (name, a) in enumerate(sorted(arrays.items(), key=lambda kv: kv[1].nbytes)):
+        share = left // (len(arrays) - n)
+        if a.nbytes > share:
+            idx = np.random.default_rng(zlib.crc32(name.encode())).choice(a.size, share // a.itemsize, replace=False)
+            a = a.reshape(-1)[np.sort(idx)]
+        left -= a.nbytes
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -247,7 +278,13 @@ def main():
     ap.add_argument("--cp", action="store_true", help="context parallelism: ONE scene per step, its views sharded over the ranks")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-gpu-torch-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the predictions of the last timed step as DIR/<name>.npy (float32, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the predictions of --impl b200")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
@@ -300,12 +337,10 @@ def main():
     dev_in = [{k: v.to(dev) for k, v in h.items()} for h in host_in]
     idx_kw = dict(depth_gt_index=list(cfg["depth_idx"]), camera_gt_index=list(cfg["cam_idx"]))
     host_out = [None] * calls
+    step_out = []
 
     def step_resident():
-        out = None
-        for c in range(calls):
-            out = model(**dev_in[c], **idx_kw)
-        return out
+        step_out[:] = [model(**dev_in[c], **idx_kw) for c in range(calls)]
 
     from omnivggt_official_b200.pipeline import StreamingPipeline
     pipe = StreamingPipeline(model, slots=2, out_keys=OUT_KEYS)
@@ -347,6 +382,8 @@ def main():
     with ClockSampler(local) as cs:
         total_ms = timed(step_resident, args.steps)
     clocks = cs.summary()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(step_out, args.dump_outputs)
     ms_step = total_ms / args.steps
     value = total_scenes * 1e3 / ms_step
 

@@ -77,6 +77,42 @@ def test_configs_follow_baseline_json():
     assert torch.allclose(R @ R.transpose(-1, -2), torch.eye(3).expand(2, 3, 3), atol=1e-5) and (torch.linalg.det(R) > 0).all()
 
 
+def test_dump_outputs_whole_and_sampled(tmp_path):
+    """--dump-outputs: one float32 .npy per returned array with the forward calls of the step concatenated, the input echo and
+    non-tensors left out; over the size cap the small arrays stay whole and the large ones become the same sample every run."""
+    import numpy as np
+    import torch
+    bench = _bench()
+    g = torch.Generator().manual_seed(0)
+
+    def call():
+        return {"pose_enc": torch.randn(2, 3, 9, generator=g), "pose_enc_list": [torch.randn(2, 3, 9, generator=g) for _ in range(2)],
+                "depth": torch.rand(2, 3, 40, 50, 1, generator=g), "world_points": torch.randn(2, 3, 40, 50, 3, generator=g).double(),
+                "images": torch.rand(2, 3, 3, 40, 50, generator=g), "view_range": (0, 3)}
+
+    outs = [call(), call()]
+    whole = {"pose_enc": torch.cat([o["pose_enc"] for o in outs]), "depth": torch.cat([o["depth"] for o in outs]),
+             "world_points": torch.cat([o["world_points"] for o in outs]).float(),
+             **{f"pose_enc_list.{i}": torch.cat([o["pose_enc_list"][i] for o in outs]) for i in range(2)}}
+    bench.dump_outputs(outs, str(tmp_path / "all"))
+    assert sorted(p.name for p in (tmp_path / "all").iterdir()) == sorted(k + ".npy" for k in whole)
+    for k, v in whole.items():
+        a = np.load(tmp_path / "all" / f"{k}.npy")
+        assert a.dtype == np.float32 and np.array_equal(a, v.numpy()), k
+
+    limit = 100_000                                     # depth 96 000 B + world_points 288 000 B + 3 x 432 B
+    for d in ("s1", "s2"):
+        bench.dump_outputs(outs, str(tmp_path / d), limit=limit)
+    got = {k: np.load(tmp_path / "s1" / f"{k}.npy") for k in whole}
+    assert sum(a.nbytes for a in got.values()) <= limit
+    for k in ("pose_enc", "pose_enc_list.0", "pose_enc_list.1"):
+        assert np.array_equal(got[k], whole[k].numpy()), k
+    for k in ("depth", "world_points"):
+        assert got[k].ndim == 1 and 0.4 * limit / 4 < got[k].size < whole[k].numel(), (k, got[k].size)
+        assert got[k].dtype == np.float32 and np.isin(got[k], whole[k].numpy()).all()
+        assert np.array_equal(got[k], np.load(tmp_path / "s2" / f"{k}.npy")), k
+
+
 def test_reference_arm_ignores_torchrun_thread_cap():
     """torchrun exports OMP_NUM_THREADS=1 to its workers; the CPU arm must still see every core."""
     # run the arm in a fresh interpreter with the caps exported and the (slow) sample stubbed
