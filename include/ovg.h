@@ -232,6 +232,10 @@ typedef struct ovg_aggregator ovg_aggregator;
 int ovg_aggregator_create(const ovg_aggregator_desc* desc, ovg_aggregator** out);
 void ovg_aggregator_destroy(ovg_aggregator* h);
 long long ovg_aggregator_workspace_bytes(const ovg_aggregator* h, int B, int S, int H, int W, int n_depth);
+/* Supported image sizes: H and W multiples of the patch size with at most OVG_MAX_PATCHES_PER_SIDE patches per side (2 044 px at
+ * patch 14), and B*S*T token rows below 2^31.  The RoPE tables then need max(H, W) / patch + 1 <= OVG_ROPE_MAX_POSITIONS rows. */
+#define OVG_MAX_PATCHES_PER_SIDE 146
+#define OVG_ROPE_MAX_POSITIONS (OVG_MAX_PATCHES_PER_SIDE + 1)
 /* patch_tokens fp32 [B*S, P, C]; inj fp32 [depth+1, B*S, C] (camera injection vectors, omnivggt_aggregator.py:172-179,:273-287);
  * depth / mask fp32 [B,S,H,W] and depth_idx device int[n_depth] (n_depth = 0: no depth aux); rope tables fp32 [maxpos, 16];
  * slots: host array of 4 device pointers, bf16 [B*S, T, 2C] each (frame half | global half); cam_out fp32 [B*S, 2C]. */

@@ -143,6 +143,7 @@ EXPORTS = {
     "ovg_runtime_attention_times": (C.c_int, [_vp, _i]),
 }
 PERCENTILE_WORKSPACE_BYTES = 6 * 8 + 512 * 4 + 4 * 4
+MAX_PATCHES_PER_SIDE = 146            # OVG_MAX_PATCHES_PER_SIDE (include/ovg.h): 2 044 px per side at patch 14
 
 
 def DEPTH_SCRATCH_DOUBLES(B: int) -> int:

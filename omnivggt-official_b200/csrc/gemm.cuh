@@ -14,7 +14,9 @@
 
 namespace ovg {
 
-enum EpiKind { EPI_BF16 = 0, EPI_RESID = 1, EPI_QKV = 2, EPI_HEADTAIL = 3 };
+// EPI_QKV_GTAB: EPI_QKV for RoPE grids above GEMM_QKV_SMEM_POS positions (cos / sin read from global memory).  A separate
+// instantiation, so that the code and register allocation of the EPI_QKV kernels do not change with it.
+enum EpiKind { EPI_BF16 = 0, EPI_RESID = 1, EPI_QKV = 2, EPI_HEADTAIL = 3, EPI_QKV_GTAB = 4 };
 enum RowMap { RM_IDENT = 0, RM_DENSE2PAD = 1, RM_PAD = 2, RM_PIXSHUF = 3 };
 
 struct GemmParams {
@@ -76,7 +78,11 @@ constexpr int GEMM_BK = 64;
 constexpr int GEMM_THREADS = 320;
 constexpr int GEMM_A_BYTES = GEMM_BM * GEMM_BK * 2;
 
-constexpr int GEMM_QKV_TABLE_BYTES = 3 * 64 * 18 * 4 + 1024;   // QKV epilogue: rope cos / sin / -sin + q,k LayerNorm affine
+// QKV epilogue: rope cos / sin / -sin for up to GEMM_QKV_SMEM_POS positions + q,k LayerNorm affine.  Larger RoPE grids
+// (images above 63 patches per side) read cos / sin from the global fp32 tables instead, so this reservation -- and with
+// it the pipeline depth of every GEMM -- does not grow with the image size.
+constexpr int GEMM_QKV_SMEM_POS = 64;
+constexpr int GEMM_QKV_TABLE_BYTES = 3 * GEMM_QKV_SMEM_POS * 18 * 4 + 1024;
 template <int BN>
 struct GemmCfg {
   static constexpr int B_BYTES = BN * GEMM_BK * 2;
@@ -120,7 +126,7 @@ __device__ __forceinline__ void epilogue_tile(const GemmParams& p, const uint32_
                                               const int colhalf, const float* s_rope, uint8_t* stg = nullptr,
                                               const CUtensorMap* tmO = nullptr, const CUtensorMap* tmO2 = nullptr,
                                               const CUtensorMap* tmO3 = nullptr) {
-  if constexpr (EPI == EPI_QKV) {
+  if constexpr (EPI == EPI_QKV || EPI == EPI_QKV_GTAB) {
     // ---- per-row RoPE position (reference omnivggt_aggregator.py:215-224; layers/rope.py:39-59)
     int py = 0, px = 0;
     {
@@ -198,7 +204,7 @@ __device__ __forceinline__ void epilogue_tile(const GemmParams& p, const uint32_
 #pragma unroll
           for (int i = 0; i < 32; ++i) v2[i] = fmul2(v2[i], qs);
         }
-        if (which < 2 && p.rope) {
+        if (EPI == EPI_QKV && which < 2 && p.rope) {
           // rotate (d, d+16) with the row angle and (32+d, 48+d) with the column angle (layers/rope.py:154-188)
 #pragma unroll
           for (int k = 0; k < 8; ++k) {
@@ -208,6 +214,24 @@ __device__ __forceinline__ void epilogue_tile(const GemmParams& p, const uint32_
             const float2 a1 = v2[16 + k], b1 = v2[24 + k];
             v2[16 + k] = ffma2(b1, nsx[k], fmul2(a1, cx[k]));
             v2[24 + k] = ffma2(a1, sx[k], fmul2(b1, cx[k]));
+          }
+        } else if (EPI == EPI_QKV_GTAB && which < 2 && p.rope) {
+          // more positions than the smem table holds: the same fp32 table entries straight from the global [maxpos][16]
+          // tables (L1 / L2 resident: 147 positions are 19 KB), -sin negated in registers -- the same operands and
+          // instructions as above, so both paths round identically
+          const float2* gcy = reinterpret_cast<const float2*>(p.rope_cos + py * 16);
+          const float2* gsy = reinterpret_cast<const float2*>(p.rope_sin + py * 16);
+          const float2* gcx = reinterpret_cast<const float2*>(p.rope_cos + px * 16);
+          const float2* gsx = reinterpret_cast<const float2*>(p.rope_sin + px * 16);
+#pragma unroll
+          for (int k = 0; k < 8; ++k) {
+            const float2 c0 = __ldg(gcy + k), s0 = __ldg(gsy + k), c1 = __ldg(gcx + k), s1 = __ldg(gsx + k);
+            const float2 a0 = v2[k], b0 = v2[8 + k];
+            v2[k] = ffma2(b0, make_float2(-s0.x, -s0.y), fmul2(a0, c0));
+            v2[8 + k] = ffma2(a0, s0, fmul2(b0, c0));
+            const float2 a1 = v2[16 + k], b1 = v2[24 + k];
+            v2[16 + k] = ffma2(b1, make_float2(-s1.x, -s1.y), fmul2(a1, c1));
+            v2[24 + k] = ffma2(a1, s1, fmul2(b1, c1));
           }
         }
         // 32 rows x 128 B (one head of 32 tokens) -> 128B-swizzled smem tile -> one bulk tensor store into the
@@ -494,8 +518,8 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
     tmem_alloc(tmem_slot, Cfg::TMEM_COLS);
     tmem_relinquish();
   }
-  if (EPI == EPI_QKV && warp >= 2) {
-    for (int i = threadIdx.x - 64; i < p.maxpos * 16; i += GEMM_THREADS - 64) {
+  if ((EPI == EPI_QKV || EPI == EPI_QKV_GTAB) && warp >= 2) {
+    for (int i = threadIdx.x - 64; EPI == EPI_QKV && i < p.maxpos * 16; i += GEMM_THREADS - 64) {   // GTAB: tables stay in global memory
       s_rope[(i >> 4) * 18 + (i & 15)] = p.rope_cos[i];
       s_rope[64 * 18 + (i >> 4) * 18 + (i & 15)] = p.rope_sin[i];
       s_rope[128 * 18 + (i >> 4) * 18 + (i & 15)] = -p.rope_sin[i];
@@ -816,7 +840,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
     if (BN == 256 && p.split_tail) tma_prefetch_desc(&tmBh);
     if (p.staged) {
       tma_prefetch_desc(&tmO);
-      if (EPI == EPI_QKV) {
+      if (EPI == EPI_QKV || EPI == EPI_QKV_GTAB) {
         tma_prefetch_desc(&tmO2);
         tma_prefetch_desc(&tmO3);
       }
@@ -835,8 +859,8 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
     tmem_alloc_2sm(tmem_slot, 2 * BN);
     tmem_relinquish_2sm();
   }
-  if (EPI == EPI_QKV && warp >= 2) {
-    for (int i = threadIdx.x - 64; i < p.maxpos * 16; i += GEMM_THREADS - 64) {
+  if ((EPI == EPI_QKV || EPI == EPI_QKV_GTAB) && warp >= 2) {
+    for (int i = threadIdx.x - 64; EPI == EPI_QKV && i < p.maxpos * 16; i += GEMM_THREADS - 64) {   // GTAB: tables stay in global memory
       s_rope[(i >> 4) * 18 + (i & 15)] = p.rope_cos[i];
       s_rope[64 * 18 + (i >> 4) * 18 + (i & 15)] = p.rope_sin[i];
       s_rope[128 * 18 + (i >> 4) * 18 + (i & 15)] = -p.rope_sin[i];

@@ -1,5 +1,6 @@
 // libovg C ABI (include/ovg.h): argument validation, TMA descriptor cache, kernel launches.
 #include <atomic>
+#include <climits>
 #include <cstdlib>
 #include <mutex>
 #include <string>
@@ -330,8 +331,8 @@ int ovg_gemm(const ovg_gemm_args* a, void* stream) {
   if (a->epi == OVG_EPI_QKV) {
     OVG_REQUIRE(a->q_out && a->bias && ((a->k_out && a->v_out) || a->n_peers > 0), "QKV args");
     if (a->qk_norm) OVG_REQUIRE(a->qn_w && a->qn_b && a->kn_w && a->kn_b, "QKV q/k norm weights");
-    if (a->rope) OVG_REQUIRE(a->rope_cos && a->rope_sin && a->maxpos > 0 && a->maxpos <= 64 && a->wp > 0,
-                             "QKV rope table (maxpos <= 64)");
+    if (a->rope) OVG_REQUIRE(a->rope_cos && a->rope_sin && a->maxpos > 0 && a->maxpos <= OVG_ROPE_MAX_POSITIONS && a->wp > 0,
+                             "QKV rope table (maxpos <= " + std::to_string(OVG_ROPE_MAX_POSITIONS) + ")");
     else p.maxpos = 0;
     OVG_REQUIRE(a->C % 64 == 0 && a->n == 3 * a->C && a->ntok > 0 && a->T > 0, "QKV geometry");
     if (p.wp <= 0) p.wp = 1;
@@ -349,6 +350,8 @@ int ovg_gemm(const ovg_gemm_args* a, void* stream) {
     if (a->rowmap != OVG_ROWS_IDENT) OVG_REQUIRE(a->gh > 0 && a->gw > 0, "row map needs gh, gw");
   }
 
+  // RoPE grids larger than the epilogue's smem table: the QKV kernels that read cos / sin from global memory
+  const bool gtab = a->epi == OVG_EPI_QKV && p.maxpos > ovg::GEMM_QKV_SMEM_POS;
   CUtensorMap ta, tb;
   int rc = get_map(a->a, a->a_cols, a->a_rows, 0, a->lda, 128, &ta);
   if (rc) return rc;
@@ -387,14 +390,16 @@ int ovg_gemm(const ovg_gemm_args* a, void* stream) {
       switch (a->epi) {
         case OVG_EPI_BF16: return launch_gemm2<256, ovg::EPI_BF16>(ta, tb, tbh, to, p, st);
         case OVG_EPI_RESID: return launch_gemm2<256, ovg::EPI_RESID>(ta, tb, tbh, to, p, st);
-        case OVG_EPI_QKV: return launch_gemm2<256, ovg::EPI_QKV>(ta, tb, tbh, to, p, st);
+        case OVG_EPI_QKV:
+          return gtab ? launch_gemm2<256, ovg::EPI_QKV_GTAB>(ta, tb, tbh, to, p, st) : launch_gemm2<256, ovg::EPI_QKV>(ta, tb, tbh, to, p, st);
         default: return fail(OVG_E_INVALID, "ovg_gemm: unknown epilogue");
       }
     }
     switch (a->epi) {
       case OVG_EPI_BF16: return launch_gemm2<128, ovg::EPI_BF16>(ta, tb, tbh, to, p, st);
       case OVG_EPI_RESID: return launch_gemm2<128, ovg::EPI_RESID>(ta, tb, tbh, to, p, st);
-      case OVG_EPI_QKV: return launch_gemm2<128, ovg::EPI_QKV>(ta, tb, tbh, to, p, st);
+      case OVG_EPI_QKV:
+        return gtab ? launch_gemm2<128, ovg::EPI_QKV_GTAB>(ta, tb, tbh, to, p, st) : launch_gemm2<128, ovg::EPI_QKV>(ta, tb, tbh, to, p, st);
       default: return fail(OVG_E_INVALID, "ovg_gemm: unknown epilogue");
     }
   }
@@ -404,7 +409,7 @@ int ovg_gemm(const ovg_gemm_args* a, void* stream) {
   switch (a->epi) {
     case OVG_EPI_BF16: return dispatch_bn<ovg::EPI_BF16>(bn, ta, tb, p, st);
     case OVG_EPI_RESID: return dispatch_bn<ovg::EPI_RESID>(bn, ta, tb, p, st);
-    case OVG_EPI_QKV: return dispatch_bn<ovg::EPI_QKV>(bn, ta, tb, p, st);
+    case OVG_EPI_QKV: return gtab ? dispatch_bn<ovg::EPI_QKV_GTAB>(bn, ta, tb, p, st) : dispatch_bn<ovg::EPI_QKV>(bn, ta, tb, p, st);
     case OVG_EPI_HEADTAIL: {
       // row-shift kernel: 3x3 taps in row-major order over a 128-channel map ((ky, kx) -> tap_off = (ky-1)*pitch + kx-1)
       bool shape_ok = a->num_taps == 9 && a->a_cols == 128 && a->n == 32;

@@ -333,8 +333,9 @@ class Engine:
         K = B * S
         hp, wp = H // self.patch, W // self.patch
         T = hp * wp + R + 1
-        if max(hp, wp) + 1 > 64:
-            raise ValueError(f"{H}x{W} input: the fused RoPE epilogue holds 64 positions per axis (at most 882 px per side)")
+        if max(hp, wp) > L.MAX_PATCHES_PER_SIDE:
+            raise ValueError(f"{H}x{W} input: at most {L.MAX_PATCHES_PER_SIDE} patches per side are supported "
+                             f"({L.MAX_PATCHES_PER_SIDE * self.patch} px at patch size {self.patch})")
         assert tuple(keep) == self.keep or set(keep) == set(self.keep), "kept layers are fixed when the engine is built"
         cos, sin = self.rope(max(hp, wp) + 1)
         Sd = len(depth_idx)
